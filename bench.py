@@ -3,7 +3,7 @@
 path on N B200s (BASELINE.json metric), with its HBM roofline, the end-to-end
 number through the C ABI with host buffers, and the CPU baseline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--cfg4]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--cfg4] [--dump-outputs DIR]
 
 One "step" = one pass of the fused kernel over one resident batch of
 BASELINE config 3: 4096 channels (1024 bridges x 4 legs) x 1640 frames of
@@ -215,15 +215,44 @@ def run_reference(args):
     }))
 
 
+DUMP_LIMIT = 64 << 20      # bytes of .npy data --dump-outputs writes at most
+
+
+def dump_frames(F, framed, fixed=()):
+    """--dump-outputs: a fixed, seeded sample of frame indices of the per-frame outputs `framed` (tensors with the
+    frame on axis 0) small enough that the whole dump stays under DUMP_LIMIT: they and the arrays `fixed` take at
+    most 4 bytes of float per byte of output, and 1 MB is set aside for frames.npy and the .npy headers."""
+    import numpy as np
+    per_frame = 4 * sum(t[0].numel() * t.element_size() for t in framed)
+    n = min(F, (DUMP_LIMIT - (1 << 20) - 4 * sum(t.numel() * t.element_size() for t in fixed)) // per_frame)
+    if n < 1:
+        raise SystemExit("--dump-outputs: one frame of the outputs is larger than the 64 MB dump")
+    return np.sort(np.random.default_rng(0).choice(F, size=n, replace=False))
+
+
+def write_dump(d, arrays):
+    """--dump-outputs: d/<name>.npy for every array, d/<name>_<field>.npy for every field of a record array
+    (padding fields skipped), in float32 or, for 32- and 64-bit integers, float64: every value exactly."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        fields = [(name, a)] if a.dtype.names is None else \
+            [(f"{name}_{f}", a[f]) for f in a.dtype.names if not f.startswith("reserved")]
+        for n, v in fields:
+            wide = v.dtype.itemsize == 8 or (v.dtype.kind in "iu" and v.dtype.itemsize == 4)
+            np.save(os.path.join(d, n + ".npy"), v.astype(np.float64 if wide else np.float32))
+
+
 def run_chain(args):
-    print(json.dumps(measure_chain(args)))
+    print(json.dumps(measure_chain(args, dump=args.dump_outputs)))
 
 
-def measure_chain(args, vp=None):
+def measure_chain(args, vp=None, dump=None):
     """--chain (and the "chain" object of the default line): SURVEY 8(d) "with RTP" accounting -- raw 180-byte ED-137 packets of every leg in, finished ED-137
     packets of every bridge out, through igd_gateway_process (receive-side walk = liveness + gate arbitration, sender
     walk on a side stream, fused decode -> meter -> mix -> encode -> packet kernel), device resident.
-    1284 algorithmic bytes per bridge-frame (4 x 180 in, 180 + 320 + 4 x 16 out)."""
+    1284 algorithmic bytes per bridge-frame (4 x 180 in, 180 + 320 + 4 x 16 out).
+    dump: directory for --dump-outputs, or None."""
     import numpy as np
     import torch
     import igate4xsoftphonedsp_b200 as ig
@@ -316,6 +345,15 @@ def measure_chain(args, vp=None):
     torch.cuda.synchronize()
     launches = vp.launch_count() - l0
     ms = e0.elapsed_time(e1) / args.steps
+    if dump:                    # what the last timed step returned and left in the four state arrays
+        fs = dump_frames(Fc, list(outs.values()), fixed=st)
+        h = {k: v[torch.from_numpy(fs).to(dev)].cpu().numpy() for k, v in outs.items()}
+        write_dump(dump, {"frames": fs, "tx_pkts": h["tx_pkts"], "tx_sizes": h["tx_sizes"].view(np.uint32),
+                          "meter": h["meter"].view(ig.METER_DT)[..., 0], "bmeter": h["bmeter"].view(ig.BRIDGE_DT),
+                          "mix": h["mix"], "rx_state": st[0].cpu().numpy().view(N.RX_STATE_DT)[:, 0],
+                          "arb_legs": st[1].cpu().numpy().view(N.ARB_LEG_DT)[:, 0],
+                          "arb_bridges": st[2].cpu().numpy().view(N.ARB_BRIDGE_DT)[:, 0],
+                          "tx_state": st[3].cpu().numpy().view(N.STATE_DT)[:, 0]})
     sampler = ClockSampler(dev.index)
     sampler.start()
     t_end = time.perf_counter() + 1.5
@@ -331,7 +369,7 @@ def measure_chain(args, vp=None):
     dummy_enc = torch.zeros((Fc, Bc, FRAME), dtype=torch.uint8, device=dev)
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
     s2 = fresh()
-    for rep in range(3):
+    for rep in range(args.steps):
         ev[0].record()
         fields, _ = vp.ed137_parse(pk.view(Fc * Cc, 180), want_payload=False)
         ev[1].record()
@@ -380,7 +418,7 @@ def measure_chain(args, vp=None):
         step(st_d, now0)
         torch.cuda.synchronize()
         ok_e2e = bool(torch.equal(h_out_t["tx_pkts"], outs["tx_pkts"].cpu()) and torch.equal(h_out_t["bmeter"], outs["bmeter"].cpu()))
-        esteps = max(2, min(args.steps, 5))
+        esteps = args.steps
         host_step(now0 + Fc * 20)
         t0 = time.perf_counter()
         for i in range(esteps):
@@ -437,7 +475,14 @@ def main():
     ap.add_argument("--serial-walks", action="store_true", help="--chain: IGD_F_WALK_SERIAL, the thread-per-channel walks (A/B)")
     ap.add_argument("--chain-bridges", type=int, default=B)
     ap.add_argument("--chain-frames", type=int, default=F)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's outputs; a fixed, seeded "
+                         "sample of frames, at most 64 MB) to DIR/<name>.npy as float32 / float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.chain:
         return run_chain(args)
     if args.cfg5:
@@ -517,6 +562,11 @@ def main():
     barrier()
     launches = vp.launch_count() - l0
     total_ms = ev[0].elapsed_time(ev[-1])
+    if args.dump_outputs and rank == 0:
+        fs = dump_frames(F, list(out.values()))
+        h = {k: v[torch.from_numpy(fs).to(dev)].cpu().numpy() for k, v in out.items()}
+        write_dump(args.dump_outputs, {"frames": fs, "mix": h["mix"], "enc": h["enc"],
+                                       "meter": h["meter"].view(ig.METER_DT)[..., 0], "bmeter": h["bmeter"].view(ig.BRIDGE_DT)})
     # clocks / throttle reasons under the same load: the K timed steps last only milliseconds, so the
     # nvidia-smi sampler (100 ms period) runs over a ~1.5 s loop of the identical kernel right after them
     clocks = None
@@ -609,7 +659,7 @@ def main():
         for t in h_out_t.values():
             t.zero_()                           # first touch while bound
         os.sched_setaffinity(0, affinity0)      # the CPU legs below use every host core again
-        esteps = max(2, min(args.steps, 5))
+        esteps = args.steps
         h2d = h_in["codes"].nbytes + h_in["gain"].nbytes + h_in["law"].nbytes + h_in["out_law"].nbytes
 
         def e2e_leg(names):
@@ -656,7 +706,7 @@ def main():
     if rank == 0 and world == 1 and not (args.cfg4 or args.cfg5 or args.no_chain) and args.frames == 1640:
         import copy
         a2 = copy.copy(args)
-        a2.no_e2e, a2.steps, a2.warmup, a2.serial_walks, a2.chain_bridges, a2.chain_frames = True, 10, 3, False, B, F
+        a2.no_e2e, a2.steps, a2.warmup, a2.serial_walks, a2.chain_bridges, a2.chain_frames = True, args.steps, 3, False, B, F
         try:
             full = measure_chain(a2, vp=vp)
             chain = {"workload": full["config"]["workload"], "value": full["value"], "unit": full["unit"],

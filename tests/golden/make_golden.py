@@ -27,6 +27,14 @@ probe oracle/_ref/libigd_ref.so):   python tests/golden/make_golden.py
                           SERVER best signal), sendR2SStatus and the
                           PTTEventDataLogger message on the seeded cases of
                           tests/rx_arb_cases.py / keepalive_cases.py
+  live_cases.json         the oracle's side of every *_live comparison of
+                          tests/test_ref_pins.py that ref_pins.json does not pin (final
+                          sender state, CSRC / extension offsets, setIncomingRTP,
+                          non-radio callback, field getters, setters, arbitration at
+                          G = 2 / 3 / 7 / 32 and with inactive legs, split-run receive
+                          state), so that they are compared without the reference build.
+                          Written by `python tests/golden/make_golden.py live_cases`, and
+                          only where those *_live tests pass against the reference
 """
 import ctypes as C
 import glob
@@ -207,5 +215,13 @@ def main():
     json.dump(ref_pins(), open(os.path.join(HERE, "ref_pins.json"), "w"), indent=1)
 
 
+def live_cases():
+    import test_ref_pins as TP
+    return TP._live_case_digest()
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["live_cases"]:
+        json.dump(live_cases(), open(os.path.join(HERE, "live_cases.json"), "w"), indent=1)
+    else:
+        main()

@@ -18,6 +18,12 @@ _DIR = os.path.join(ROOT, "oracle", "_ref")
 
 SERVER, CLIENT = 1, 2
 
+# what the reference's encode_sdp (TransportAdapter.cpp:941-1044) wrote for a radio call of type "Rxonly" and
+# keep-alive period 150, and its slave-transport counters after attach + two encode_sdp calls
+SDP_RXONLY_150 = ("rtphe:1\ntype:Rxonly\ntxrxmode:TRx\nbss:RSSI\nsigtime:1\nptt_rep:0\n"
+                  "R2S-KeepAlivePeriod:150\nR2S-KeepAliveMultiplier:10\n")
+COUNTERS_ATTACH, COUNTERS_ENCODE_SDP = 4 + 1, 4 + 7
+
 
 class State(C.Structure):
     _fields_ = [("radiostatus", C.c_int), ("pttstatus", C.c_int), ("sqlstatus", C.c_int),

@@ -169,8 +169,21 @@ def test_sendR2SStatus_through_shim_equals_reference():
                 wsz[t, c] = n
                 want[t, c, :n] = out[:n]
             Rf.refta_destroy(h)
-    else:
-        pytest.skip("needs oracle/_ref (the oracle walk has no send history form)")
+    else:                                                        # the same moves on the oracle's adapters
+        L = O.lib()
+        _, _, _, ads = T.run_oracle(s)                           # the three send_rtp ticks of the history
+        want = np.zeros((60, 24, 20), np.uint8)
+        wsz = np.zeros((60, 24), np.uint32)
+        out = np.zeros(512, np.uint8)
+        for c, a in enumerate(ads):
+            for t in range(60):
+                k = ctl[t, c]
+                L.orc_setAdapterPtt(C.byref(a), int(k["pttstatus"]), int(k["pttpriority"]), int(k["callRecorder"]))
+                L.orc_setAdapterQslOn(C.byref(a), int(k["sqlstatus"]), 0, int(k["ed137_bssi"]))
+                L.orc_setAdapterPttId(C.byref(a), int(k["pttid"]))
+                n = L.orc_sendR2SStatus(C.byref(a), now0 + t * tick, out.ctypes.data)
+                wsz[t, c] = n
+                want[t, c, :n] = out[:n]
     for bankwide in (False, True):
         bank = S.shimta_open(0, 24)
         hs = []
@@ -240,6 +253,8 @@ def test_vtable_layout_passthrough_sdp_and_channel_reuse():
         Rf.refta_counters(rh, rcnt)
         assert list(cnt) == list(rcnt)
         Rf.refta_destroy(rh)
+    assert sdp_rxonly == RP.SDP_RXONLY_150
+    assert cnt[RP.COUNTERS_ATTACH] == 1 and cnt[RP.COUNTERS_ENCODE_SDP] == 2
     assert bits == 0b0111_0111_0001
     assert "ptt-id:1\n" in sdp_trx and "ptt-id" not in sdp_rxonly and "R2S-KeepAlivePeriod:150\n" in sdp_rxonly
     rtcp = np.zeros(8, np.uint8)

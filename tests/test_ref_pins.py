@@ -9,7 +9,10 @@ them: tp->op->send_rtp, the RTP callback registered in tp->op->attach, the publi
                  compare arrays (they run wherever oracle/_ref/ is present: the build container and, since
                  the .so travels with gpurun, the GPU box);
   golden tests   compare the oracle with tests/golden/ref_pins.json, which tests/golden/make_golden.py
-                 wrote FROM THE REFERENCE RUN (they need nothing but the oracle).
+                 wrote FROM THE REFERENCE RUN (they need nothing but the oracle), and with
+                 tests/golden/live_cases.json: the oracle's side of the remaining *_live comparisons, recorded
+                 where they pass, so that a change to the oracle or to the shared cases is caught without the
+                 reference build.
 """
 import ctypes as C
 import hashlib
@@ -337,14 +340,13 @@ def test_reference_vtable_and_sdp_live():
     assert Rf.refta_vtable_passthrough(h) == 0b0111_0111_0001
     buf = C.create_string_buffer(1024)
     Rf.refta_encode_sdp(h, buf, 1024)
-    assert buf.value.decode() == ("rtphe:1\ntype:Rxonly\ntxrxmode:TRx\nbss:RSSI\nsigtime:1\nptt_rep:0\n"
-                                  "R2S-KeepAlivePeriod:150\nR2S-KeepAliveMultiplier:10\n")
+    assert buf.value.decode() == RP.SDP_RXONLY_150
     Rf.refta_setCallType(h, b"TRx")
     Rf.refta_encode_sdp(h, buf, 1024)
     assert "ptt-id:1\n" in buf.value.decode()
     cnt = (C.c_int * 16)()
     Rf.refta_counters(h, cnt)
-    assert cnt[4 + 1] == 1 and cnt[4 + 7] == 2          # attach once, encode_sdp twice reached the slave
+    assert cnt[RP.COUNTERS_ATTACH] == 1 and cnt[RP.COUNTERS_ENCODE_SDP] == 2    # attach once, encode_sdp twice
     Rf.refta_destroy(h)
 
 
@@ -370,6 +372,100 @@ def _oracle_digest():
     out["event_messages"] = [_oracle_event_message(*_event_case(seed)[:2], b"sip:radio1@10.0.0.5", 3)[0]
                              for seed in (1, 2, 3)]
     return out
+
+
+def _live_case_digest():
+    """the oracle's side of every *_live comparison above that ref_pins.json does not already pin, on the same cases
+    (tests/golden/make_golden.py live_cases -> live_cases.json)"""
+    out = {"tx_final_state": {}}
+    for s in T.SCENARIOS:
+        _, _, _, ads = T.run_oracle(s)
+        out["tx_final_state"][s["name"]] = [
+            {**{f: int(getattr(a, f)) for f in RP.TX_STATE_FIELDS}, "send_pkt_buff": sha(np.frombuffer(bytes(a.send_pkt_buff), np.uint8)),
+             "tmp_payload_buf": sha(np.frombuffer(bytes(a.tmp_payload_buf), np.uint8)), "send_payload_bufSize": int(a.send_payload_bufSize)}
+            for a, leg in zip(ads, s["legs"]) if leg["radiocall"]]
+    pk, sz, bm, _ = T.run_oracle(T.SCENARIOS[0], signed_char=1)
+    out["tx_signed_char_sizes"] = sha(sz)
+    rng = np.random.default_rng(4)                  # test_send_rtp_csrc_extension_padding_live
+    out["csrc"] = []
+    o = np.zeros(512, np.uint8)
+    for cc, x, extw in ((0, 0, 0), (2, 0, 0), (0, 1, 1), (1, 1, 2), (3, 0, 0)):
+        pkt = np.zeros(12 + 4 * cc + (4 + 4 * extw if x else 0) + 160, np.uint8)
+        pkt[:] = rng.integers(0, 256, pkt.size)
+        pkt[0] = 0x80 | (x << 4) | cc
+        pkt[1] = 8
+        if x:
+            pkt[12 + 4 * cc + 2] = 0
+            pkt[12 + 4 * cc + 3] = extw
+        a = O.Adapter()
+        L.orc_adapter_init(C.byref(a), 1, 0, b"TRx", 200, 5000)
+        L.orc_setAdapterPtt(C.byref(a), 1, 3, 0)
+        n = L.orc_transport_send_rtp(C.byref(a), pkt.ctypes.data, pkt.size, 5000, o.ctypes.data, 1, 0)
+        out["csrc"].append({"size": int(n), "packet": sha(o[:n]), "OutgoingRTP": int(a.OutgoingRTP)})
+    pkts, sizes, present = R.make_rx_stream(120, 8, seed=9)    # test_rtp_cb_state_carry_live
+    out["rx_state_carry"] = sha(R.oracle_rx_walk(pkts, R.ref_comparable_sizes(sizes), present)[1])
+    out["setIncomingRTP"] = {}
+    for signed_char in (0, 1):                      # test_setIncomingRTP_bytemean_live
+        rng = np.random.default_rng(21)
+        a = O.Adapter()
+        L.orc_adapter_init(C.byref(a), 1, 0, b"TRx", 200, 0)
+        hdr = np.zeros(20, np.uint8)
+        res = []
+        for n in (160, 164, 24, 1, 80, 256, 200):
+            pkt = rng.integers(0, 256, 20 + n, dtype=np.uint8)
+            if n == 80:
+                pkt[20:] = rng.integers(128, 256, n)
+            L.orc_hdr_write(hdr.ctypes.data, 2, 0, 1, 0, 0, 8, 1, 160, 9, 0x0167, 1, 0x10013178)
+            pkt[:20] = hdr
+            r = L.orc_transport_rtp_cb(C.byref(a), pkt.ctypes.data, pkt.size, 40, 1, signed_char)
+            res.append({"n": n, "forwarded": int(r), "IncomingRTP": int(a.IncomingRTP), "payload_bufSize": int(a.payload_bufSize),
+                        "payload": sha(np.frombuffer(bytes(a.payload_buff), np.uint8)[:n])})
+        out["setIncomingRTP"][str(signed_char)] = res
+    rng = np.random.default_rng(2)                  # test_non_radio_rtp_cb_live
+    pkt = rng.integers(0, 256, 172, dtype=np.uint8)
+    pkt[0], pkt[1] = 0x80, 8
+    a = O.Adapter()
+    L.orc_adapter_init(C.byref(a), 0, 0, b"", 200, 0)
+    r = L.orc_transport_rtp_cb(C.byref(a), pkt.ctypes.data, 172, 0, 0, 0)
+    out["non_radio"] = {"forwarded": int(r), "payload_bufSize": int(a.payload_bufSize), "ed137_value": int(a.ed137_value),
+                        "payload": sha(np.frombuffer(bytes(a.payload_buff), np.uint8)[:160])}
+    rng = np.random.default_rng(8)                  # test_field_getters_oracle_equals_reference_live
+    words = [0, 1, 0x00013100, 0x000131C0, 0x00013140, 0x00013180, 0x00413100, 0x104131F8, 0xE0013100,
+             0x10013178, 0xFFFFFFFF] + [int(x) for x in rng.integers(0, 2**32, 200)]
+    f = O.Fields()
+    got = []
+    for w in words:
+        L.orc_ed137_fields_from_word(w, C.byref(f))
+        got.append([f.bss, f.ptt_type, f.ptt_id, f.squelch, f.active])
+    out["field_getters"] = sha(np.array(got, np.int64))
+    a = O.Adapter()                                 # test_setters_by_call_id_live
+    L.orc_adapter_init(C.byref(a), 1, 0, b"TRx", 200, 0)
+    L.orc_setAdapterPtt(C.byref(a), 1, 3, 1)
+    L.orc_setAdapterQslOn(C.byref(a), 1, 2, 1000 >> 6)
+    L.orc_setTxRxSlaveEnable(C.byref(a), 1, 0)
+    out["setters"] = {f: int(getattr(a, f)) for f in ("pttstatus", "pttpriority", "callRecorder", "sqlstatus", "sqlpriority",
+                                                       "ed137_bssi", "rxSlaveEnableChanged", "txSlaveEnableChanged",
+                                                       "trxSlaveEnableChangedCount")}
+    out["arbitration"] = {}
+    for mode, G, seed in ((N.ARB_CLIENT_PTT, 4, 4), (N.ARB_SERVER_BEST, 4, 4), (N.ARB_CLIENT_PTT, 7, 1),
+                          (N.ARB_CLIENT_PTT, 32, 2), (N.ARB_SERVER_BEST, 2, 3), (N.ARB_SERVER_BEST, 3, 5)):
+        g, lg, br = R.oracle_arb_walk(R.make_arb_words(200, 6, G, mode, seed=seed), G, mode)
+        out["arbitration"][f"mode{mode}_G{G}_seed{seed}"] = {"gain": sha(g), "legs": sha(lg), "bridges": sha(br)}
+    rng = np.random.default_rng(12)                 # test_gate_arbitration_inactive_legs_live
+    for mode in (N.ARB_CLIENT_PTT, N.ARB_SERVER_BEST):
+        active = (rng.random(20) < 0.7).astype(np.uint8)
+        g, lg, br = R.oracle_arb_walk(R.make_arb_words(150, 5, 4, mode, seed=17), 4, mode, active=active)
+        out["arbitration"][f"mode{mode}_inactive"] = {"gain": sha(g), "legs": sha(lg), "bridges": sha(br)}
+    return out
+
+
+def test_oracle_matches_the_live_cases_pins(golden_dir):
+    """every *_live comparison on a machine without the reference build: the oracle against what it computed on the
+    same cases where the *_live tests showed it equal to the reference"""
+    g = json.load(open(os.path.join(golden_dir, "live_cases.json")))
+    got = _live_case_digest()
+    for k in got:
+        assert got[k] == g[k], k
 
 
 def test_oracle_matches_goldens_generated_from_the_reference(golden_dir):
