@@ -37,6 +37,10 @@ cudaError_t igd_k_ed137_parse(const igd_launch_cfg &c, const uint8_t *pkts, cons
                               uint8_t *payload_out);
 cudaError_t igd_k_ed137_pack(const igd_launch_cfg &c, const igd_ed137_pack_desc &d,
                              igd_tx_plan_rec *plan, int32_t *last_src);
+// igd_gateway_fanout: the sender walk over d.C = B*G legs (d.payload NULL), then k_fanout_tile encodes pcm [F][B][160]
+// into every leg's packet (d.bytemean_out may be NULL); two launches
+cudaError_t igd_k_gateway_fanout(const igd_launch_cfg &c, const igd_ed137_pack_desc &d, int G, const int16_t *pcm,
+                                 const uint8_t *law, igd_tx_plan_rec *plan, int32_t *last_src);
 cudaError_t igd_k_ed137_keepalive(const igd_launch_cfg &c, uint8_t *hdr20, igd_ed137_state *state, size_t C,
                                   long long now, uint32_t *sizes);
 // the walks with the tick axis across the lanes of a warp (igd_walks.cuh / igd_walks.cu)

@@ -843,6 +843,45 @@ __global__ void __launch_bounds__(256) k_ed137_assemble(const igd_ed137_pack_des
     }
 }
 
+// The two tile kernels below (k_ed137_assemble_tile, k_fanout_tile) build 64 wire packets in a shared-memory
+// image of 64 x 45 words and share its header rewrite and its write-out.
+//
+// Header rewrite of transport_send_rtp (TransportAdapter.cpp:715-725, 800): PJSIP's 12 bytes h0..h2 with x = 1, the
+// plan's marker and PT 123, then the profile / length word and the ED-137 word -- the packet's first five words.
+__device__ __forceinline__ void tile_header(uint32_t *o, const igd_tx_plan_rec &r, uint32_t h0, uint32_t h1, uint32_t h2)
+{
+    uint32_t v0 = h0 | 0x10u;                                              // x = 1 (:725)
+    v0 = (v0 & ~0x8000u) | ((r.flags & 2u) ? 0x8000u : 0u);                // m (:715-723)
+    if (r.flags & 1u) v0 = (v0 & ~0x7F00u) | (123u << 8);                  // pt = 123
+    o[0] = v0; o[1] = h1; o[2] = h2; o[3] = 0x01006701u; o[4] = bswap32(r.word);   // 0x0167, 0x0001 big-endian; htonl (:800)
+}
+
+// Write-out of a finished image of np packets to dst (= packet 0 of the tile): ONE bulk async store (TMA) when the
+// image holds every byte of the tile (*partial == 0: every packet is 180 bytes, or the image is zero past each packet's
+// size), otherwise coalesced word stores of only the bytes each packet's size covers, the rest of its slot zero.
+// Called by every thread of the CTA once the image and size_s are written.
+__device__ __forceinline__ void tile_store(uint8_t *dst, const uint32_t *img, const uint32_t *size_s, uint32_t np,
+                                           const uint32_t *partial)
+{
+    fence_proxy_async();             // the image is read by the async proxy below
+    __syncthreads();
+    const uint32_t tile_bytes = np * IGD_PKT_MAX;
+    if (!*partial && (tile_bytes & 15u) == 0 && (reinterpret_cast<uintptr_t>(dst) & 15u) == 0) {
+        if (threadIdx.x == 0) {
+            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
+                         ::"l"(dst), "r"(shared_addr(img)), "r"(tile_bytes) : "memory");
+            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");     // smem must outlive the read
+        }
+    } else {
+        uint32_t *out = reinterpret_cast<uint32_t *>(dst);
+        for (uint32_t w = threadIdx.x; w < np * kPktWords; w += blockDim.x) {
+            const uint32_t p = w / kPktWords, k = w - p * kPktWords;
+            out[w] = 4 * k < size_s[p] ? img[w] : 0u;              // past the packet the slot reads zero
+        }
+    }
+}
+
 // Tile form of the assembly for the wire shape (out_stride 180, 160-byte payloads): a CTA builds
 // 64 packets in shared memory (headers by 64 threads, payload chunks by all threads with 16-byte
 // loads) and writes the image out with coalesced word stores, only the bytes each packet's size
@@ -878,11 +917,7 @@ __global__ void __launch_bounds__(256) k_ed137_assemble_tile(const igd_ed137_pac
         const igd_tx_plan_rec r = plan[i];
         const uint32_t *hdr = reinterpret_cast<const uint32_t *>(d.rtp12 + i * 12);
         const uint32_t h0 = hdr[0], h1 = hdr[1], h2 = hdr[2];
-        uint32_t v0 = h0 | 0x10u;                                              // x = 1 (:725)
-        v0 = (v0 & ~0x8000u) | ((r.flags & 2u) ? 0x8000u : 0u);                // m (:715-723)
-        if (r.flags & 1u) v0 = (v0 & ~0x7F00u) | (123u << 8);                  // pt = 123
-        uint32_t *o = img + p * kPktWords;
-        o[0] = v0; o[1] = h1; o[2] = h2; o[3] = 0x01006701u; o[4] = bswap32(r.word);
+        tile_header(img + p * kPktWords, r, h0, h1, h2);
         size_s[p] = r.size;
         srcf_s[p] = r.src_frame;
         flag_s[p] = r.flags;
@@ -925,28 +960,96 @@ __global__ void __launch_bounds__(256) k_ed137_assemble_tile(const igd_ed137_pac
             atomicAdd(&bsum_s[p], bs);
         }
     }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // the image is read by the async proxy below
-    __syncthreads();
-    const uint32_t tile_bytes = np * IGD_PKT_MAX;
-    if (!not_full && (tile_bytes & 15u) == 0 && (reinterpret_cast<uintptr_t>(d.pkts) & 15u) == 0) {
-        // every packet of the tile is a full 180-byte audio packet: ONE bulk async store (TMA) writes the image
-        if (threadIdx.x == 0) {
-            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
-                         ::"l"(d.pkts + first * IGD_PKT_MAX), "r"(shared_addr(img)), "r"(tile_bytes) : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");     // smem must outlive the read
-        }
-    } else {
-        uint32_t *out = reinterpret_cast<uint32_t *>(d.pkts + first * IGD_PKT_MAX);
-        for (uint32_t w = threadIdx.x; w < np * kPktWords; w += blockDim.x) {
-            const uint32_t p = w / kPktWords, k = w - p * kPktWords;
-            out[w] = 4 * k < size_s[p] ? img[w] : 0u;              // past the packet the slot reads zero
-        }
-    }
+    tile_store(d.pkts + first * IGD_PKT_MAX, img, size_s, np, &not_full);
     if (threadIdx.x < np) {
         const uint32_t p = threadIdx.x;
         const bool audio = size_s[p] != 0 && !(flag_s[p] & 1u);
         d.bytemean_out[first + p] = audio ? (uint8_t)igd_bytemean_from_sum(bsum_s[p], IGD_FRAME) : (uint8_t)0;
+    }
+}
+
+// ============================================================ gateway fan-out
+// igd_gateway_fanout's assembly: the same 64-packet tile as k_ed137_assemble_tile, its payloads encoded here from the
+// bridges' PCM instead of read.  Packet i = f*B*G + b*G + g belongs to bridge-frame i / G, so a tile's 64 packets span
+// at most ceil(63/G)+1 consecutive bridge-frames (G = 1: 64) whose PCM is one contiguous run: ONE bulk async copy
+// stages it.  Every (bridge-frame, law) present among the tile's legs is encoded once (16 samples per thread, the
+// packed compressor of igd_g711_encode_ch), its byte sum taken once for the level of every packet that carries it,
+// and the 16 code bytes go into the payload of each of those packets that is sent whole (180 bytes).  The image is
+// zero past each packet's size, so every tile of whole packets leaves with ONE bulk store, whatever its sizes (with
+// word stores for the mixed tiles, which are most of them, the kernel ran at 37 % of the HBM peak).
+constexpr int kFanBf = kPktTile;         // bridge-frames a tile can touch: ceil(63/G)+1 <= 64
+__host__ __device__ constexpr uint32_t fanout_tile_bfs(int G) { return (uint32_t)((kPktTile - 2 + G) / G + 1); }
+// 32 registers, no spills: eight CTAs per SM (19 KB of shared memory each at G = 4) keep more tiles' loads and stores
+// in flight than the six that 40 registers allowed
+__global__ void __launch_bounds__(256, 8) k_fanout_tile(const igd_ed137_pack_desc d, const int G,
+                                                     const int16_t *__restrict__ pcm, const uint8_t *__restrict__ law,
+                                                     const igd_tx_plan_rec *__restrict__ plan)
+{
+    __shared__ __align__(128) uint32_t img[kPktTile * kPktWords];             // the 64 packets being built
+    extern __shared__ __align__(128) uint32_t pcm_s[];                       // the tile's bridge-frames (fanout_tile_bfs(G))
+    __shared__ unsigned long long legs_s[2 * kFanBf];   // [bridge-frame][law]: bit p = packet p of the tile carries it
+    __shared__ int bsum_s[2 * kFanBf];                  // [bridge-frame][law]: byte sum of the encoded frame
+    __shared__ uint64_t bar;
+    __shared__ uint32_t size_s[kPktTile];
+    __shared__ uint32_t pair_s[kPktTile];               // packet p -> its [bridge-frame][law] entry; bit 31 = PT 123
+    const size_t npkts = (size_t)d.F * d.C;
+    const size_t first = (size_t)blockIdx.x * kPktTile;
+    const uint32_t np = (uint32_t)min((size_t)kPktTile, npkts - first);
+    const size_t bf0 = first / (uint32_t)G;
+    const uint32_t nbf = (uint32_t)((first + np - 1) / (uint32_t)G - bf0) + 1;
+    const bool sc = (d.flags & IGD_F_SIGNED_CHAR) != 0;
+    const uint32_t bar_s = shared_addr(&bar);
+    if (threadIdx.x == 0) {
+        mbar_init(bar_s, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_expect_tx(bar_s, nbf * IGD_FRAME * 2);
+        bulk_g2s(shared_addr(pcm_s), pcm + bf0 * IGD_FRAME, nbf * IGD_FRAME * 2, bar_s);
+    }
+    for (uint32_t k = threadIdx.x; k < 2 * nbf; k += blockDim.x) { legs_s[k] = 0ull; bsum_s[k] = 0; }
+    __syncthreads();                 // barrier initialised, leg masks cleared
+    if (threadIdx.x < np) {
+        const uint32_t p = threadIdx.x;
+        const size_t i = first + p;
+        const igd_tx_plan_rec r = plan[i];
+        const uint32_t *hdr = reinterpret_cast<const uint32_t *>(d.rtp12 + i * 12);
+        tile_header(img + p * kPktWords, r, hdr[0], hdr[1], hdr[2]);
+        size_s[p] = r.size;
+        d.sizes[i] = r.size;
+        const size_t c = i % (size_t)d.C;                                     // leg b*G + g
+        const uint32_t pr = 2u * (uint32_t)(i / (uint32_t)G - bf0) + (law[c] != 0 ? 1u : 0u);   // igd_enc_law_make: 0 = A-law, else u-law
+        pair_s[p] = pr | ((r.flags & 1u) << 31);
+        atomicOr(&legs_s[pr], 1ull << p);
+    }
+    __syncthreads();                 // leg masks and headers complete
+    for (uint32_t w = threadIdx.x; w < np * kPktWords; w += blockDim.x) {     // zero past each packet (no payload there)
+        const uint32_t p = w / kPktWords;
+        if (4 * (w - p * kPktWords) >= size_s[p]) img[w] = 0u;
+    }
+    mbar_wait(bar_s, 0);             // the PCM has landed
+    for (uint32_t j = threadIdx.x; j < 2 * nbf * kChunks; j += blockDim.x) {
+        const uint32_t pr = j / kChunks, ch = j - pr * kChunks;
+        const unsigned long long m = legs_s[pr];
+        if (!m) continue;            // no leg of this bridge-frame in the tile uses this law
+        const uint4 *src = reinterpret_cast<const uint4 *>(pcm_s + (pr >> 1) * (IGD_FRAME / 2) + ch * 8);
+        const uint4 a = src[0], b = src[1];
+        const uint32_t pk[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+        const uint4 e = encode16_packed(pk, enc_pk_make((int)(pr & 1u)));
+        int bs = 0;
+        bs = bytesum4(e.x, sc, bs); bs = bytesum4(e.y, sc, bs); bs = bytesum4(e.z, sc, bs); bs = bytesum4(e.w, sc, bs);
+        atomicAdd(&bsum_s[pr], bs);
+        for (unsigned long long mm = m; mm; mm &= mm - 1) {
+            const uint32_t p = (uint32_t)(__ffsll((long long)mm) - 1);
+            if (size_s[p] != IGD_PKT_MAX) continue;
+            uint32_t *o = img + p * kPktWords + 5 + ch * 4;
+            o[0] = e.x; o[1] = e.y; o[2] = e.z; o[3] = e.w;
+        }
+    }
+    const uint32_t whole = 0u;       // the image holds every byte of the tile
+    tile_store(d.pkts + first * IGD_PKT_MAX, img, size_s, np, &whole);
+    if (threadIdx.x < np && d.bytemean_out) {
+        const uint32_t p = threadIdx.x, pr = pair_s[p];
+        const bool audio = size_s[p] != 0 && !(pr >> 31);          // setOutgoingRTP (roip_ed137.cpp:6500-6536), clean
+        d.bytemean_out[first + p] = audio ? (uint8_t)igd_bytemean_from_sum(bsum_s[pr & 0x7FFFFFFFu], IGD_FRAME) : (uint8_t)0;
     }
 }
 
@@ -1113,6 +1216,16 @@ cudaError_t igd_k_ed137_pack(const igd_launch_cfg &c, const igd_ed137_pack_desc 
     e = cudaGetLastError();
     if (e != cudaSuccess || !d.stale_payload) return e;
     k_ed137_stale_update<<<grid_for(c, (size_t)d.C * 32, 256, 8), 256, 0, c.stream>>>(d, last_src);
+    return cudaGetLastError();
+}
+
+cudaError_t igd_k_gateway_fanout(const igd_launch_cfg &c, const igd_ed137_pack_desc &d, int G, const int16_t *pcm,
+                                 const uint8_t *law, igd_tx_plan_rec *plan, int32_t *last_src)
+{
+    cudaError_t e = igd_k_ed137_plan(c, d, plan, last_src);
+    if (e != cudaSuccess) return e;
+    const size_t tiles = ((size_t)d.F * d.C + kPktTile - 1) / kPktTile;
+    k_fanout_tile<<<(unsigned)tiles, 256, fanout_tile_bfs(G) * IGD_FRAME * 2, c.stream>>>(d, G, pcm, law, plan);
     return cudaGetLastError();
 }
 

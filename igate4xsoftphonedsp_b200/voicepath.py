@@ -508,6 +508,44 @@ class VoicePath:
         self._chk(self._lib.igd_gateway_process(self._h, C.byref(d)))
         return o
 
+    def gateway_fanout(self, pcm, law, tx_rtp12, tx_state, tx_ctl=None, now_ms0=0, tick_ms=20, flags=0, level=True,
+                       out=None):
+        """The other direction of a bridge (igd_gateway_fanout): one PCM frame per bridge and tick in, a finished
+        ED-137 packet for every leg of the bridge out, each encoded in its leg's law and sent with its leg's sender
+        state.  pcm int16 [F][B][160]; law u8 [B*G]; tx_rtp12 u8 [F][B*G][12]; tx_ctl [F][B*G] or None; tx_state
+        STATE_DT [B*G] is updated in place.  Returns dict(tx_pkts [F][B*G][180], tx_sizes [F][B*G]) plus tx_level
+        [F][B*G] when `level`; `out` (such a dict) is written instead of fresh buffers, e.g. inside a CUDA graph."""
+        mem = self._mode(pcm, law, tx_rtp12, tx_state, tx_ctl)
+        F, B, n = pcm.shape
+        Cn = law.numel() if _is_torch(law) else np.size(law)
+        if n != N.FRAME or B == 0 or Cn % B:
+            raise IgdError("pcm must be [F][B][160] and law [B*G]")
+        G = Cn // B
+        if tuple(tx_rtp12.shape[:2]) != (F, Cn):
+            raise IgdError("tx_rtp12 must be [F][B*G][12]")
+        keys = ("tx_pkts", "tx_sizes") + (("tx_level",) if level else ())
+        if mem == N.MEM_DEVICE:
+            dev = pcm.device
+            mk = {"tx_pkts": lambda: torch.empty((F, Cn, N.PKT_MAX), dtype=torch.uint8, device=dev),
+                  "tx_sizes": lambda: torch.empty((F, Cn), dtype=torch.int32, device=dev),
+                  "tx_level": lambda: torch.empty((F, Cn), dtype=torch.uint8, device=dev)}
+        else:
+            pcm = np.ascontiguousarray(pcm, dtype=np.int16)
+            law = np.ascontiguousarray(law, dtype=np.uint8)
+            tx_rtp12 = np.ascontiguousarray(tx_rtp12, dtype=np.uint8)
+            if tx_state.dtype != N.STATE_DT or not tx_state.flags.c_contiguous:
+                raise IgdError("tx_state must be a contiguous STATE_DT array (updated in place)")
+            if tx_ctl is not None:
+                tx_ctl = np.ascontiguousarray(tx_ctl, dtype=N.CTL_DT)
+            mk = {"tx_pkts": lambda: np.empty((F, Cn, N.PKT_MAX), np.uint8), "tx_sizes": lambda: np.empty((F, Cn), np.uint32),
+                  "tx_level": lambda: np.empty((F, Cn), np.uint8)}
+        o = out if out is not None else {k: mk[k]() for k in keys}
+        d = N.FanoutDesc(C.sizeof(N.FanoutDesc), mem, F, B, G, int(flags), int(tick_ms), 0, int(now_ms0),
+                         self._ptr(pcm), self._ptr(law), self._ptr(tx_rtp12), self._ptr(tx_ctl), self._ptr(tx_state),
+                         self._ptr(o["tx_pkts"]), self._ptr(o["tx_sizes"]), self._ptr(o.get("tx_level")))
+        self._chk(self._lib.igd_gateway_fanout(self._h, C.byref(d)))
+        return o
+
     # ------------------------------------------------------------ recorder
     def wav_image(self, payload, rate=8000, law=N.LAW_ULAW, ref_quirks=False):
         """WavWriter file image (header + body) built on the GPU."""

@@ -524,6 +524,48 @@ typedef struct {
 } igd_gateway_desc;
 int igd_gateway_process(igd_ctx *ctx, const igd_gateway_desc *d);
 
+/* ------------------------------------------------- gateway fan-out: one frame per bridge in, a packet per leg out
+ * The other direction of a bridge.  In the reference every call port is connected to conference slot 0
+ * (roip_ed137.cpp:4907-4920), so on each 20 ms tick every call of the bridge sends the same slot-0 frame (the
+ * sound-device capture), G.711-encoded in that call's own codec and sent through transport_send_rtp
+ * (TransportAdapter.cpp:635-874) with that call's own ED-137 sender state (PTT, squelch, keep-alive throttle, marker,
+ * RRC word).  One call does this for F ticks of B bridges x G legs, leg c = b*G + g:
+ *   in : pcm      [F][B][160]    the frame every leg of bridge b sends on tick f
+ *        law      [B*G]          IGD_LAW_* of each leg's call
+ *        tx_rtp12 [F][B*G][12]   PJSIP-built RTP headers; tx_ctl [F][B*G] setter values or NULL
+ *   out: tx_pkts  [F][B*G][180]  the bytes of a slot past tx_sizes are zero
+ *        tx_sizes [F][B*G]       0 = suppressed by the keep-alive throttle, 20 = keep-alive, 180 = audio
+ *        tx_level [F][B*G]       optional: setOutgoingRTP level (roip_ed137.cpp:6500-6536), 0 for PT 123 / nothing sent
+ *   tx_state [B*G] is updated in place.
+ * The results are byte for byte those of igd_g711_encode_ch over pcm with each bridge's frame copied to its G legs,
+ * followed by igd_ed137_pack (payload_len 160, out_stride 180, stale_payload NULL, flags & IGD_F_SIGNED_CHAR) --
+ * except tx_state.rtpFalse, the reference's never-read stuck-audio counter, which is not maintained here (as in
+ * igd_gateway_process: the payload it looks at is encoded after the sender walk).  Quirks Q2 / Q3 are not offered:
+ * flags other than IGD_F_SIGNED_CHAR are IGD_EINVAL.  Two kernels: the sender walk and one that stages the PCM,
+ * encodes each bridge-frame once per law among its legs and assembles the packets; no code array exists between
+ * them.  Device pointers: pcm and tx_pkts 16-byte aligned, tx_state and tx_ctl 8, tx_rtp12 and tx_sizes 4.  The
+ * device form only enqueues work on the context's stream and, once an earlier call of the same or a larger shape has
+ * sized the scratch, allocates nothing: it can be captured into a CUDA graph.
+ * Algorithmic bytes per bridge-frame: 320 + G*12 + G*180 (G = 4: 1088).                                      */
+typedef struct {
+    uint32_t struct_size;        /* = sizeof(igd_fanout_desc)                     */
+    int32_t mem;                 /* IGD_MEM_DEVICE or IGD_MEM_HOST (all pointers) */
+    int32_t F, B, G;             /* 1 <= G <= IGD_MAX_LEGS; leg c = b*G + g        */
+    uint32_t flags;              /* IGD_F_SIGNED_CHAR only                        */
+    int32_t tick_ms;             /* 20                                            */
+    int32_t reserved;
+    int64_t now_ms0;             /* currenttime of tick f = now_ms0 + f*tick_ms    */
+    const int16_t *pcm;          /* [F][B][160] the frame every leg of bridge b sends (conference slot 0) */
+    const uint8_t *law;          /* [B*G] IGD_LAW_* of each leg's call            */
+    const uint8_t *tx_rtp12;     /* [F][B*G][12] PJSIP-built RTP headers          */
+    const igd_ed137_ctl *tx_ctl; /* [F][B*G] setter values per tick, or NULL      */
+    igd_ed137_state *tx_state;   /* [B*G] in/out                                  */
+    uint8_t *tx_pkts;            /* [F][B*G][180]; bytes past tx_sizes are zero   */
+    uint32_t *tx_sizes;          /* [F][B*G] 0 = suppressed, 20 = keep-alive, 180 */
+    uint8_t *tx_level;           /* [F][B*G] optional: setOutgoingRTP level, 0 for PT 123 / nothing sent */
+} igd_fanout_desc;
+int igd_gateway_fanout(igd_ctx *ctx, const igd_fanout_desc *d);
+
 /* ------------------------------------------------------------ recorder sink
  * replaces: WavWriter::start/wav_write/stop (WavWriter.cpp:63-156).
  * Builds the complete file image on the GPU: 44-byte header + body.
