@@ -115,6 +115,14 @@ class FanoutDesc(C.Structure):
                 ("tx_state", C.c_void_p), ("tx_pkts", C.c_void_p), ("tx_sizes", C.c_void_p), ("tx_level", C.c_void_p)]
 
 
+class FanoutPktDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("mem", C.c_int32), ("F", C.c_int32), ("B", C.c_int32), ("G", C.c_int32),
+                ("flags", C.c_uint32), ("tick_ms", C.c_int32), ("reserved", C.c_int32), ("now_ms0", C.c_int64),
+                ("rx_pkts", C.c_void_p), ("rx_sizes", C.c_void_p), ("in_law", C.c_void_p), ("law", C.c_void_p),
+                ("tx_rtp12", C.c_void_p), ("tx_ctl", C.c_void_p), ("tx_state", C.c_void_p), ("tx_pkts", C.c_void_p),
+                ("tx_sizes", C.c_void_p), ("tx_level", C.c_void_p)]
+
+
 class ArbDesc(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("mem", C.c_int32), ("F", C.c_int32), ("B", C.c_int32),
                 ("G", C.c_int32), ("mode", C.c_int32), ("word_stride", C.c_uint32), ("flags", C.c_uint32),
@@ -161,6 +169,7 @@ SYMBOLS = {
     "igd_gate_arbitrate": (_i, [_vp, C.POINTER(ArbDesc)]),
     "igd_gateway_process": (_i, [_vp, C.POINTER(GatewayDesc)]),
     "igd_gateway_fanout": (_i, [_vp, C.POINTER(FanoutDesc)]),
+    "igd_gateway_fanout_packets": (_i, [_vp, C.POINTER(FanoutPktDesc)]),
     "igd_wav_size": (_sz, [_sz, _i]),
     "igd_wav_image": (_i, [_vp, _vp, _sz, _i, _i, _i, _vp, C.POINTER(_sz), _i]),
     "igd_wav_images": (_i, [_vp, _vp, _sz, _sz, _vp, _sz, _vp, _i, _i, _vp, _sz, _i]),

@@ -1211,6 +1211,61 @@ int igd_gateway_fanout(igd_ctx *c, const igd_fanout_desc *d)
     return finish(c, mem);
 }
 
+// ---------------------------------------------------------------- gateway fan-out from the console call's packets
+int igd_gateway_fanout_packets(igd_ctx *c, const igd_fanout_pkt_desc *d)
+{
+    if (!c || !d || d->struct_size != sizeof(igd_fanout_pkt_desc))
+        return fail(c, IGD_EINVAL, "igd_gateway_fanout_packets: bad descriptor");
+    if (d->F < 0 || d->B < 0 || d->G < 1 || d->G > IGD_MAX_LEGS || (d->flags & ~IGD_F_SIGNED_CHAR))
+        return fail(c, IGD_EINVAL, "igd_gateway_fanout_packets: bad shape (1 <= G <= 32) or flags (IGD_F_SIGNED_CHAR only)");
+    if (d->F == 0 || d->B == 0) return IGD_OK;
+    if ((int64_t)d->B * d->G > INT32_MAX) return fail(c, IGD_EINVAL, "igd_gateway_fanout_packets: B*G exceeds 2^31 legs");
+    if (!d->rx_pkts || !d->in_law || !d->law || !d->tx_rtp12 || !d->tx_state || !d->tx_pkts || !d->tx_sizes)
+        return fail(c, IGD_EINVAL, "igd_gateway_fanout_packets: null buffer");
+    const int mem = d->mem;
+    if (mem == IGD_MEM_DEVICE &&
+        (!aligned(d->rx_pkts, 16) || !aligned(d->tx_pkts, 16) || !aligned(d->tx_state, 8) ||
+         (d->tx_ctl && !aligned(d->tx_ctl, 8)) || !aligned(d->tx_rtp12, 4) || !aligned(d->tx_sizes, 4) ||
+         (d->rx_sizes && !aligned(d->rx_sizes, 4))))
+        return fail(c, IGD_EINVAL, "igd_gateway_fanout_packets: misaligned device pointer (rx_pkts / tx_pkts 16 bytes; "
+                                   "tx_state / tx_ctl 8; tx_rtp12 / tx_sizes / rx_sizes 4)");
+    IGD_BIND(c);
+    const size_t F = d->F, B = d->B, Cn = B * d->G, n = F * Cn;
+    igd_ed137_pack_desc k;
+    memset(&k, 0, sizeof k);
+    k.struct_size = sizeof k; k.mem = IGD_MEM_DEVICE; k.F = d->F; k.C = (int32_t)Cn; k.flags = d->flags;
+    k.payload_len = IGD_FRAME; k.out_stride = IGD_PKT_MAX; k.tick_ms = d->tick_ms; k.now_ms0 = d->now_ms0;
+    k.payload = nullptr;             // the sender walk runs before the payloads exist (rtpFalse is not maintained)
+    int rc;
+    const uint8_t *drx, *dinlaw, *dlaw;
+    const uint32_t *drsz = nullptr;
+    if ((rc = in_arg(c, mem, 0, d->tx_rtp12, n * 12, &k.rtp12))) return rc;
+    if ((rc = in_arg(c, mem, 1, d->rx_pkts, F * B * IGD_PKT_MAX, &drx))) return rc;
+    if (d->tx_ctl && (rc = in_arg(c, mem, 2, d->tx_ctl, n, &k.ctl))) return rc;
+    {
+        const igd_ed137_state *tmp = nullptr;
+        if ((rc = in_arg(c, mem, 3, d->tx_state, Cn, &tmp))) return rc;
+        k.state = const_cast<igd_ed137_state *>(tmp);
+    }
+    if ((rc = out_arg(c, mem, 4, d->tx_pkts, n * IGD_PKT_MAX, &k.pkts))) return rc;
+    if ((rc = out_arg(c, mem, 5, d->tx_sizes, n, &k.sizes))) return rc;
+    if (d->tx_level && (rc = out_arg(c, mem, 6, d->tx_level, n, &k.bytemean_out))) return rc;
+    if ((rc = in_arg(c, mem, 7, d->law, Cn, &dlaw))) return rc;
+    if (d->rx_sizes && (rc = in_arg(c, mem, 10, d->rx_sizes, F * B, &drsz))) return rc;
+    if ((rc = in_arg(c, mem, 11, d->in_law, B, &dinlaw))) return rc;
+    void *dplan, *dlast;             // the slots igd_ed137_pack keeps its plan in
+    if ((rc = scratch(c, 8, n * sizeof(igd_tx_plan_rec), &dplan))) return rc;
+    if ((rc = scratch(c, 9, Cn * sizeof(int32_t), &dlast))) return rc;
+    IGD_CUDA(c, igd_k_gateway_fanout_packets(cfg_of(c), k, d->G, drx, drsz, dinlaw, dlaw,
+                                             static_cast<igd_tx_plan_rec *>(dplan), static_cast<int32_t *>(dlast)));
+    c->launches += 2;
+    if ((rc = out_done(c, mem, d->tx_pkts, k.pkts, n * IGD_PKT_MAX))) return rc;
+    if ((rc = out_done(c, mem, d->tx_sizes, k.sizes, n))) return rc;
+    if (d->tx_level && (rc = out_done(c, mem, d->tx_level, k.bytemean_out, n))) return rc;
+    if ((rc = out_done(c, mem, d->tx_state, k.state, Cn))) return rc;
+    return finish(c, mem);
+}
+
 // ---------------------------------------------------------------- recorder
 size_t igd_wav_size(size_t payload_bytes, int ref_quirks)
 {

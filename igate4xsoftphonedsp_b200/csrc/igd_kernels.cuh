@@ -41,6 +41,11 @@ cudaError_t igd_k_ed137_pack(const igd_launch_cfg &c, const igd_ed137_pack_desc 
 // into every leg's packet (d.bytemean_out may be NULL); two launches
 cudaError_t igd_k_gateway_fanout(const igd_launch_cfg &c, const igd_ed137_pack_desc &d, int G, const int16_t *pcm,
                                  const uint8_t *law, igd_tx_plan_rec *plan, int32_t *last_src);
+// igd_gateway_fanout_packets: the same sender walk, then k_fanout_pkt_tile maps the console packets rx_pkts [F][B][180]
+// (rx_sizes [F][B] or NULL = all 180, in_law [B]) into every leg's packet; two launches
+cudaError_t igd_k_gateway_fanout_packets(const igd_launch_cfg &c, const igd_ed137_pack_desc &d, int G,
+                                         const uint8_t *rx_pkts, const uint32_t *rx_sizes, const uint8_t *in_law,
+                                         const uint8_t *law, igd_tx_plan_rec *plan, int32_t *last_src);
 cudaError_t igd_k_ed137_keepalive(const igd_launch_cfg &c, uint8_t *hdr20, igd_ed137_state *state, size_t C,
                                   long long now, uint32_t *sizes);
 // the walks with the tick axis across the lanes of a warp (igd_walks.cuh / igd_walks.cu)

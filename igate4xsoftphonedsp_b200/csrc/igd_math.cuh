@@ -92,6 +92,16 @@ IGD_HD uint32_t igd_g711_enc1(int x, const igd_enc_law &L)
     return code ^ (s ? L.mneg : L.mpos);
 }
 
+// ---------------------------------------------------------------- G.711 transcode
+// The code that a G.711 code of in_law becomes once decoded and encoded again in out_law (0 = A-law, else u-law):
+// enc_out(dec_in(code)).  A-law -> A-law is the identity, u-law -> u-law the identity but for 0x7F (-0) -> 0xFF (+0).
+// k_fanout_pkt_tile builds its 2 x 2 x 256 code table from this.
+IGD_HD uint32_t igd_g711_transcode1(uint32_t code, int in_law, int out_law)
+{
+    const int x = in_law ? igd_ulaw2lin(code) : igd_alaw2lin(code);
+    return igd_g711_enc1(x, igd_enc_law_make(out_law));
+}
+
 // ---------------------------------------------------------------- meters
 // rms_dbfs = 10 log10(S/160) - 20 log10(32768); peak_dbfs = 20 log10(P/32768).
 // log2 through the SFU (abs error ~2^-22) and the affine map in fp32: total

@@ -1053,6 +1053,136 @@ __global__ void __launch_bounds__(256, 8) k_fanout_tile(const igd_ed137_pack_des
     }
 }
 
+// ============================================================ gateway fan-out from packets
+// igd_gateway_fanout_packets' assembly: k_fanout_tile's tile, with each payload mapped code by code out of the console
+// call's received packet instead of encoded from PCM.  Bridge-frame bf's console packet is rx_pkts + bf*180, so a tile's
+// bridge-frames are again one contiguous run.  bf0*180 is only 4-byte aligned, so ONE bulk async copy stages the
+// 16-byte-aligned window that covers the run, and the run starts `lead` = 0, 1, 2 or 3 words into it: payload words in
+// shared memory are 4-byte aligned and read as 32-bit words.  The window never leaves the array: when the array's size
+// is not a multiple of 16, the last tile's copy stops at the last whole 16 bytes and threads load the <= 3 words after.
+// Every output byte is enc_out(dec_in(code)): a 2 x 2 x 256 code table [in law][out law][code] from igd_g711_transcode1,
+// built per CTA (one code per thread, four entries) while the staging copy and the plan loads are in flight.  A table
+// in device memory would be context state that must exist before a graph capture, to save work that is hidden anyway.
+// A bridge-frame whose console packet is not a whole G.711 audio frame (the IGD_RXE_FRAME rule: fields_of_header,
+// then igd_fields_no_audio) sends digital silence: the out law's code for PCM 0.
+__host__ __device__ constexpr uint32_t fanout_pkt_stage_bytes(int G)      // lead + the bridge-frames' packets, to 16 B
+{
+    return (12u + fanout_tile_bfs(G) * IGD_PKT_MAX + 15u) & ~15u;         // G = 1: 11 536, G = 4: 3072, G = 32: 560
+}
+__global__ void __launch_bounds__(256, 8) k_fanout_pkt_tile(const igd_ed137_pack_desc d, const int G,
+                                                         const uint8_t *__restrict__ rx_pkts,
+                                                         const uint32_t *__restrict__ rx_sizes,
+                                                         const uint8_t *__restrict__ in_law, const uint8_t *__restrict__ law,
+                                                         const igd_tx_plan_rec *__restrict__ plan)
+{
+    __shared__ __align__(128) uint32_t img[kPktTile * kPktWords];             // the 64 packets being built
+    extern __shared__ __align__(128) uint32_t win_s[];                       // the staged window (fanout_pkt_stage_bytes(G))
+    __shared__ unsigned long long legs_s[2 * kFanBf];   // [bridge-frame][law]: bit p = packet p of the tile carries it
+    __shared__ int bsum_s[2 * kFanBf];                  // [bridge-frame][law]: byte sum of the mapped frame
+    __shared__ __align__(4) uint8_t tab_s[2 * 2 * 256];  // [in law][out law][code] -> code
+    __shared__ uint32_t rsz_s[kFanBf];                  // [bridge-frame]: received size of the console packet
+    __shared__ uint32_t bfi_s[kFanBf];                  // [bridge-frame]: bit 0 = in law is u-law, bit 1 = no audio frame
+    __shared__ uint64_t bar;
+    __shared__ uint32_t size_s[kPktTile];
+    __shared__ uint32_t pair_s[kPktTile];               // packet p -> its [bridge-frame][law] entry; bit 31 = PT 123
+    const size_t npkts = (size_t)d.F * d.C;
+    const size_t first = (size_t)blockIdx.x * kPktTile;
+    const uint32_t np = (uint32_t)min((size_t)kPktTile, npkts - first);
+    const size_t bf0 = first / (uint32_t)G;
+    const uint32_t nbf = (uint32_t)((first + np - 1) / (uint32_t)G - bf0) + 1;
+    const bool sc = (d.flags & IGD_F_SIGNED_CHAR) != 0;
+    // the run [run0, run1) of console-packet bytes and the window [w0, w1) that stages it
+    const size_t run0 = bf0 * IGD_PKT_MAX, run1 = run0 + (size_t)nbf * IGD_PKT_MAX;
+    const size_t w0 = run0 & ~(size_t)15;
+    const size_t w1 = min((run1 + 15) & ~(size_t)15, (npkts / (uint32_t)G * IGD_PKT_MAX) & ~(size_t)15);
+    const uint32_t lead = (uint32_t)(run0 - w0) / 4;
+    const uint32_t bar_s = shared_addr(&bar);
+    if (threadIdx.x == 0) {
+        mbar_init(bar_s, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_expect_tx(bar_s, (uint32_t)(w1 - w0));
+        bulk_g2s(shared_addr(win_s), rx_pkts + w0, (uint32_t)(w1 - w0), bar_s);
+    }
+    if (run1 > w1 && threadIdx.x < (uint32_t)(run1 - w1) / 4)      // the array's last words, past its last whole 16 bytes
+        win_s[(w1 - w0) / 4 + threadIdx.x] = reinterpret_cast<const uint32_t *>(rx_pkts + w1)[threadIdx.x];
+#pragma unroll
+    for (int k = 0; k < 4; k++)                          // blockDim.x == 256: thread t maps code t for every law pair
+        tab_s[k * 256 + threadIdx.x] = (uint8_t)igd_g711_transcode1(threadIdx.x, k >> 1, k & 1);
+    for (uint32_t k = threadIdx.x; k < 2 * nbf; k += blockDim.x) { legs_s[k] = 0ull; bsum_s[k] = 0; }
+    __syncthreads();                 // barrier initialised, leg masks cleared
+    if (threadIdx.x < np) {
+        const uint32_t p = threadIdx.x;
+        const size_t i = first + p;
+        const igd_tx_plan_rec r = plan[i];
+        const uint32_t *hdr = reinterpret_cast<const uint32_t *>(d.rtp12 + i * 12);
+        tile_header(img + p * kPktWords, r, hdr[0], hdr[1], hdr[2]);
+        size_s[p] = r.size;
+        d.sizes[i] = r.size;
+        const size_t c = i % (size_t)d.C;                                     // leg b*G + g
+        const uint32_t pr = 2u * (uint32_t)(i / (uint32_t)G - bf0) + (law[c] != 0 ? 1u : 0u);   // igd_enc_law_make: 0 = A-law, else u-law
+        pair_s[p] = pr | ((r.flags & 1u) << 31);
+        atomicOr(&legs_s[pr], 1ull << p);
+        if (p < nbf) {               // nbf <= np: the console packet's size and its call's law
+            const size_t bf = bf0 + p;
+            rsz_s[p] = rx_sizes ? rx_sizes[bf] : (uint32_t)IGD_PKT_MAX;
+            bfi_s[p] = in_law[bf % (size_t)((uint32_t)d.C / (uint32_t)G)] != 0 ? 1u : 0u;
+        }
+    }
+    __syncthreads();                 // leg masks, headers and bridge-frame records complete
+    for (uint32_t w = threadIdx.x; w < np * kPktWords; w += blockDim.x) {     // zero past each packet (no payload there)
+        const uint32_t p = w / kPktWords;
+        if (4 * (w - p * kPktWords) >= size_s[p]) img[w] = 0u;
+    }
+    mbar_wait(bar_s, 0);             // the console packets have landed
+    if (threadIdx.x < nbf) {         // transport_rtp_cb's view of the console packet (the navail guard of k_rxarb_bridge)
+        const uint32_t k = threadIdx.x, size = rsz_s[k];
+        const uint32_t *hw = win_s + lead + k * kPktWords;
+        const uint32_t navail = min(size, (uint32_t)IGD_PKT_MAX) / 4;
+        const igd_ed137_fields fl = fields_of_header(navail > 0 ? hw[0] : 0u, navail > 3 ? hw[3] : 0u, navail > 4 ? hw[4] : 0u, size);
+        const uint4 fw = *reinterpret_cast<const uint4 *>(&fl);
+        if (igd_fields_no_audio(fw.y, fw.z, fw.w)) bfi_s[k] |= 2u;
+    }
+    __syncthreads();                 // no-audio flags complete
+    // unit j = (pair, chunk ch): payload words ch, ch + 10, ch + 20, ch + 30, so that neighbouring lanes read and
+    // write neighbouring words
+    for (uint32_t j = threadIdx.x; j < 2 * nbf * kChunks; j += blockDim.x) {
+        const uint32_t pr = j / kChunks, ch = j - pr * kChunks;
+        const unsigned long long m = legs_s[pr];
+        if (!m) continue;            // no leg of this bridge-frame in the tile uses this law
+        const uint32_t info = bfi_s[pr >> 1], o = pr & 1u;
+        uint32_t e[4];
+        if (info & 2u) {             // silence: the table's entry for u-law 0xFF, which decodes to PCM 0
+            const uint32_t s = tab_s[(2u + o) * 256u + 0xFFu] * 0x01010101u;
+            e[0] = s; e[1] = s; e[2] = s; e[3] = s;
+        } else {
+            const uint8_t *tb = tab_s + ((info & 1u) * 2u + o) * 256u;
+            const uint32_t *src = win_s + lead + (pr >> 1) * kPktWords + 5 + ch;
+#pragma unroll
+            for (int q = 0; q < 4; q++) {
+                const uint32_t w = src[q * kChunks];
+                e[q] = __byte_perm(__byte_perm(tb[w & 0xFFu], tb[(w >> 8) & 0xFFu], 0x0040),
+                                   __byte_perm(tb[(w >> 16) & 0xFFu], tb[w >> 24], 0x0040), 0x5410);
+            }
+        }
+        int bs = 0;
+        bs = bytesum4(e[0], sc, bs); bs = bytesum4(e[1], sc, bs); bs = bytesum4(e[2], sc, bs); bs = bytesum4(e[3], sc, bs);
+        atomicAdd(&bsum_s[pr], bs);
+        for (unsigned long long mm = m; mm; mm &= mm - 1) {
+            const uint32_t p = (uint32_t)(__ffsll((long long)mm) - 1);
+            if (size_s[p] != IGD_PKT_MAX) continue;
+            uint32_t *o4 = img + p * kPktWords + 5 + ch;
+            o4[0] = e[0]; o4[kChunks] = e[1]; o4[2 * kChunks] = e[2]; o4[3 * kChunks] = e[3];
+        }
+    }
+    const uint32_t whole = 0u;       // the image holds every byte of the tile
+    tile_store(d.pkts + first * IGD_PKT_MAX, img, size_s, np, &whole);
+    if (threadIdx.x < np && d.bytemean_out) {
+        const uint32_t p = threadIdx.x, pr = pair_s[p];
+        const bool audio = size_s[p] != 0 && !(pr >> 31);          // setOutgoingRTP (roip_ed137.cpp:6500-6536), clean
+        d.bytemean_out[first + p] = audio ? (uint8_t)igd_bytemean_from_sum(bsum_s[pr & 0x7FFFFFFFu], IGD_FRAME) : (uint8_t)0;
+    }
+}
+
 // ============================================================ recorder sink
 __global__ void k_wav_image(const uint8_t *__restrict__ payload, size_t n, int rate, int law, int ref_quirks,
                             uint8_t *__restrict__ out)
@@ -1226,6 +1356,18 @@ cudaError_t igd_k_gateway_fanout(const igd_launch_cfg &c, const igd_ed137_pack_d
     if (e != cudaSuccess) return e;
     const size_t tiles = ((size_t)d.F * d.C + kPktTile - 1) / kPktTile;
     k_fanout_tile<<<(unsigned)tiles, 256, fanout_tile_bfs(G) * IGD_FRAME * 2, c.stream>>>(d, G, pcm, law, plan);
+    return cudaGetLastError();
+}
+
+cudaError_t igd_k_gateway_fanout_packets(const igd_launch_cfg &c, const igd_ed137_pack_desc &d, int G,
+                                         const uint8_t *rx_pkts, const uint32_t *rx_sizes, const uint8_t *in_law,
+                                         const uint8_t *law, igd_tx_plan_rec *plan, int32_t *last_src)
+{
+    cudaError_t e = igd_k_ed137_plan(c, d, plan, last_src);
+    if (e != cudaSuccess) return e;
+    const size_t tiles = ((size_t)d.F * d.C + kPktTile - 1) / kPktTile;
+    k_fanout_pkt_tile<<<(unsigned)tiles, 256, fanout_pkt_stage_bytes(G), c.stream>>>(d, G, rx_pkts, rx_sizes, in_law, law,
+                                                                                    plan);
     return cudaGetLastError();
 }
 

@@ -546,6 +546,51 @@ class VoicePath:
         self._chk(self._lib.igd_gateway_fanout(self._h, C.byref(d)))
         return o
 
+    def gateway_fanout_packets(self, rx_pkts, in_law, law, tx_rtp12, tx_state, rx_sizes=None, tx_ctl=None, now_ms0=0,
+                               tick_ms=20, flags=0, level=True, out=None):
+        """gateway_fanout with slot 0 as received from the console call (igd_gateway_fanout_packets): the console's
+        ED-137 packets in, a finished packet for every leg of the bridge out.  rx_pkts u8 [F][B][180] as received;
+        rx_sizes u32 [F][B] or None (all 180); in_law u8 [B] the console call's law; law u8 [B*G]; tx_rtp12 u8
+        [F][B*G][12]; tx_ctl [F][B*G] or None; tx_state STATE_DT [B*G] is updated in place.  Every leg of bridge b
+        sends the G.711 frame of rx_pkts[f][b] decoded in in_law[b], or digital silence where that packet is not a
+        whole audio frame.  Returns dict(tx_pkts [F][B*G][180], tx_sizes [F][B*G]) plus tx_level [F][B*G] when
+        `level`; `out` (such a dict) is written instead of fresh buffers, e.g. inside a CUDA graph."""
+        mem = self._mode(rx_pkts, in_law, law, tx_rtp12, tx_state, rx_sizes, tx_ctl)
+        F, B, n = rx_pkts.shape
+        Cn = law.numel() if _is_torch(law) else np.size(law)
+        nin = in_law.numel() if _is_torch(in_law) else np.size(in_law)
+        if n != N.PKT_MAX or B == 0 or Cn % B or nin != B:
+            raise IgdError("rx_pkts must be [F][B][180], in_law [B] and law [B*G]")
+        G = Cn // B
+        if tuple(tx_rtp12.shape[:2]) != (F, Cn):
+            raise IgdError("tx_rtp12 must be [F][B*G][12]")
+        keys = ("tx_pkts", "tx_sizes") + (("tx_level",) if level else ())
+        if mem == N.MEM_DEVICE:
+            dev = rx_pkts.device
+            mk = {"tx_pkts": lambda: torch.empty((F, Cn, N.PKT_MAX), dtype=torch.uint8, device=dev),
+                  "tx_sizes": lambda: torch.empty((F, Cn), dtype=torch.int32, device=dev),
+                  "tx_level": lambda: torch.empty((F, Cn), dtype=torch.uint8, device=dev)}
+        else:
+            rx_pkts = np.ascontiguousarray(rx_pkts, dtype=np.uint8)
+            if rx_sizes is not None:
+                rx_sizes = np.ascontiguousarray(rx_sizes, dtype=np.uint32)
+            in_law = np.ascontiguousarray(in_law, dtype=np.uint8)
+            law = np.ascontiguousarray(law, dtype=np.uint8)
+            tx_rtp12 = np.ascontiguousarray(tx_rtp12, dtype=np.uint8)
+            if tx_state.dtype != N.STATE_DT or not tx_state.flags.c_contiguous:
+                raise IgdError("tx_state must be a contiguous STATE_DT array (updated in place)")
+            if tx_ctl is not None:
+                tx_ctl = np.ascontiguousarray(tx_ctl, dtype=N.CTL_DT)
+            mk = {"tx_pkts": lambda: np.empty((F, Cn, N.PKT_MAX), np.uint8), "tx_sizes": lambda: np.empty((F, Cn), np.uint32),
+                  "tx_level": lambda: np.empty((F, Cn), np.uint8)}
+        o = out if out is not None else {k: mk[k]() for k in keys}
+        d = N.FanoutPktDesc(C.sizeof(N.FanoutPktDesc), mem, F, B, G, int(flags), int(tick_ms), 0, int(now_ms0),
+                            self._ptr(rx_pkts), self._ptr(rx_sizes), self._ptr(in_law), self._ptr(law),
+                            self._ptr(tx_rtp12), self._ptr(tx_ctl), self._ptr(tx_state), self._ptr(o["tx_pkts"]),
+                            self._ptr(o["tx_sizes"]), self._ptr(o.get("tx_level")))
+        self._chk(self._lib.igd_gateway_fanout_packets(self._h, C.byref(d)))
+        return o
+
     # ------------------------------------------------------------ recorder
     def wav_image(self, payload, rate=8000, law=N.LAW_ULAW, ref_quirks=False):
         """WavWriter file image (header + body) built on the GPU."""

@@ -566,6 +566,51 @@ typedef struct {
 } igd_fanout_desc;
 int igd_gateway_fanout(igd_ctx *ctx, const igd_fanout_desc *d);
 
+/* ------------------------------------------------- gateway fan-out from packets: the console call's packets in, a packet per leg out
+ * igd_gateway_fanout with slot 0 taken from where a gateway without a sound card has it: the remote console, whose
+ * audio arrives as ED-137 packets on the same call that igd_gateway_process sends the bridge's mix out on (a call has
+ * one codec in both directions, so in_law is igd_gateway_process's out_law).  One call does F ticks of B bridges x G
+ * legs, leg c = b*G + g:
+ *   in : rx_pkts  [F][B][180]    the console call's packets as received, zero padded
+ *        rx_sizes [F][B]         received sizes, 0 = nothing arrived; NULL = all 180
+ *        in_law   [B]            IGD_LAW_* of the console call
+ *        law, tx_rtp12, tx_ctl   as in igd_fanout_desc
+ *   out: tx_pkts, tx_sizes, tx_level, tx_state as in igd_fanout_desc
+ * The frame every leg of bridge b sends on tick f is igd_g711_decode of bytes 20..179 of rx_pkts[f][b] in in_law[b]
+ * when that packet carries a whole G.711 audio frame -- accepted PT 0 or 8, payload_len 160, not dropped (the
+ * IGD_RXE_FRAME rule; the decode law is in_law, not the packet's PT, as in igd_process_packets) -- and digital silence
+ * (PCM 0) otherwise: a keep-alive, a lost, short or PT 18 packet, an unaccepted PT.  The results are byte for byte
+ * those of igd_ed137_parse (payload_out) -> igd_g711_decode_ch in in_law -> PCM 0 on the ticks without a whole frame
+ * -> igd_gateway_fanout with that PCM: packets, sizes, levels and tx_state, except tx_state.rtpFalse, which is not
+ * maintained (as in igd_gateway_fanout).  No PCM exists in between: each payload byte is mapped through a 256-entry
+ * code table of the (in law, leg law) pair.  1 <= G <= 32; flags other than IGD_F_SIGNED_CHAR are IGD_EINVAL;
+ * B*G <= 2^31.  Two kernels: the sender walk and one that stages the console packets, maps each bridge-frame once per
+ * law among its legs and assembles the packets.  Device pointers: rx_pkts and tx_pkts 16-byte aligned, tx_state and
+ * tx_ctl 8, tx_rtp12, tx_sizes and rx_sizes 4.  The device form only enqueues work on the context's stream and, once
+ * an earlier call of the same or a larger shape has sized the scratch, allocates nothing: it can be captured into a
+ * CUDA graph together with igd_gateway_process.
+ * Algorithmic bytes per bridge-frame: 180 + G*12 + G*180 (G = 4: 948, against 1088 for igd_gateway_fanout).     */
+typedef struct {
+    uint32_t struct_size;        /* = sizeof(igd_fanout_pkt_desc)                 */
+    int32_t mem;                 /* IGD_MEM_DEVICE or IGD_MEM_HOST (all pointers) */
+    int32_t F, B, G;             /* 1 <= G <= IGD_MAX_LEGS; leg c = b*G + g        */
+    uint32_t flags;              /* IGD_F_SIGNED_CHAR only                        */
+    int32_t tick_ms;             /* 20                                            */
+    int32_t reserved;
+    int64_t now_ms0;             /* currenttime of tick f = now_ms0 + f*tick_ms    */
+    const uint8_t *rx_pkts;      /* [F][B][180] the console call's packets as received (zero padded) */
+    const uint32_t *rx_sizes;    /* [F][B] received sizes, 0 = nothing arrived; NULL = all 180 */
+    const uint8_t *in_law;       /* [B] IGD_LAW_* of the console call             */
+    const uint8_t *law;          /* [B*G] IGD_LAW_* of each leg's call            */
+    const uint8_t *tx_rtp12;     /* [F][B*G][12] PJSIP-built RTP headers          */
+    const igd_ed137_ctl *tx_ctl; /* [F][B*G] setter values per tick, or NULL      */
+    igd_ed137_state *tx_state;   /* [B*G] in/out                                  */
+    uint8_t *tx_pkts;            /* [F][B*G][180]; bytes past tx_sizes are zero   */
+    uint32_t *tx_sizes;          /* [F][B*G] 0 = suppressed, 20 = keep-alive, 180 */
+    uint8_t *tx_level;           /* [F][B*G] optional: setOutgoingRTP level, 0 for PT 123 / nothing sent */
+} igd_fanout_pkt_desc;
+int igd_gateway_fanout_packets(igd_ctx *ctx, const igd_fanout_pkt_desc *d);
+
 /* ------------------------------------------------------------ recorder sink
  * replaces: WavWriter::start/wav_write/stop (WavWriter.cpp:63-156).
  * Builds the complete file image on the GPU: 44-byte header + body.
