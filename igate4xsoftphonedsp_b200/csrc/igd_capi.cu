@@ -485,7 +485,12 @@ int fused_job_host(igd_ctx *c, const FusedJob &j)
     if (j.meter && (rc = scratch(c, 6, nbuf * fc * C * sizeof(igd_meter_rec), &dmeter))) return rc;
     if (j.bmeter && (rc = scratch(c, 7, nbuf * fc * B * sizeof(igd_bridge_rec), &dbm))) return rc;
     cudaStream_t sin = c->copy_streams[0], sout = c->copy_streams[1];
-    // ev[0..1]: input of buffer i ready; ev[2..3]: kernel on buffer i done; ev[4..5]: output drained
+    // ev[0..1]: input of buffer i ready; ev[2..3]: kernel on buffer i done; ev[4..5]: output drained; ev[6]: fork.
+    // The copy-in stream starts after the work already queued on the caller's stream: the device form of another call
+    // may still be reading slots 2, 3 or 8 there (igd_gateway_process keeps its gains in slot 8, the fan-outs their
+    // sender plan), and scratch() only synchronizes when a slot grows.
+    IGD_CUDA(c, cudaEventRecord(c->ev[6], c->stream));
+    IGD_CUDA(c, cudaStreamWaitEvent(sin, c->ev[6], 0));
     bool out_pending[2] = {false, false};
     auto chunk = [&](size_t ch) -> int {
         const int i = (int)(ch % nbuf);
@@ -792,7 +797,7 @@ int igd_ed137_keepalive(igd_ctx *c, uint8_t *hdr20, igd_ed137_state *state, size
 int igd_rx_track(igd_ctx *c, const igd_rx_track_desc *d)
 {
     if (!c || !d || d->struct_size != sizeof(igd_rx_track_desc)) return fail(c, IGD_EINVAL, "igd_rx_track: bad descriptor");
-    if (d->F < 0 || d->C < 0 || d->wd_ticks < 0) return fail(c, IGD_EINVAL, "igd_rx_track: bad shape");
+    if (d->F < 0 || d->C < 0 || d->wd_ticks < 0 || d->frame0 < 0) return fail(c, IGD_EINVAL, "igd_rx_track: bad shape / frame0");
     if (d->F == 0 || d->C == 0) return IGD_OK;
     if (!d->fields || !d->state || !d->events) return fail(c, IGD_EINVAL, "igd_rx_track: null buffer");
     const int mem = d->mem;
@@ -861,9 +866,12 @@ int igd_gateway_process(igd_ctx *c, const igd_gateway_desc *d)
 {
     if (!c || !d || d->struct_size != sizeof(igd_gateway_desc))
         return fail(c, IGD_EINVAL, "igd_gateway_process: bad descriptor");
-    if (d->F < 0 || d->B < 0 || d->wd_ticks < 0 || (d->arb_mode != IGD_ARB_CLIENT_PTT && d->arb_mode != IGD_ARB_SERVER_BEST))
-        return fail(c, IGD_EINVAL, "igd_gateway_process: bad shape / mode");
+    if (d->F < 0 || d->B < 0 || d->wd_ticks < 0 || d->frame0 < 0 ||
+        (d->arb_mode != IGD_ARB_CLIENT_PTT && d->arb_mode != IGD_ARB_SERVER_BEST))
+        return fail(c, IGD_EINVAL, "igd_gateway_process: bad shape / mode / frame0");
     if (d->G != 4) return fail(c, IGD_EINVAL, "igd_gateway_process: G must be 4");
+    if (d->flags & ~(IGD_F_SIGNED_CHAR | IGD_F_KERNEL_W | IGD_F_WALK_SERIAL))
+        return fail(c, IGD_EINVAL, "igd_gateway_process: flags (IGD_F_SIGNED_CHAR, IGD_F_KERNEL_W, IGD_F_WALK_SERIAL only)");
     if (d->F == 0 || d->B == 0) return IGD_OK;
     if (!d->rx_pkts || !d->law || !d->rx_state || !d->arb_legs || !d->arb_bridges || !d->out_law || !d->tx_rtp12 ||
         !d->tx_state || !d->tx_pkts || !d->tx_sizes)

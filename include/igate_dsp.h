@@ -407,7 +407,8 @@ typedef struct {
     int32_t r2s_period_ms;       /* radio->r2sPeriod, default 200 (roip_ed137.h:685) */
     int32_t wd_ticks;            /* the watchdog runs on every wd_ticks-th frame
                                     (40 ms timer / 20 ms frames = 2); 0 = never    */
-    int32_t frame0;              /* index of this call's first frame (watchdog phase) */
+    int32_t frame0;              /* index of this call's first frame (watchdog phase),
+                                    >= 0 (negative: IGD_EINVAL)                    */
     int64_t now_ms0;
     const igd_ed137_fields *fields;   /* [F][C] from igd_ed137_parse               */
     const uint8_t *present;      /* [F][C] 0 = no packet on that tick; NULL = all  */
@@ -491,12 +492,13 @@ typedef struct {
     uint32_t struct_size;        /* = sizeof(igd_gateway_desc)                    */
     int32_t mem;                 /* IGD_MEM_DEVICE or IGD_MEM_HOST (all pointers) */
     int32_t F, B, G;
-    uint32_t flags;              /* IGD_F_SIGNED_CHAR, IGD_F_KERNEL_W, IGD_F_WALK_SERIAL */
+    uint32_t flags;              /* IGD_F_SIGNED_CHAR, IGD_F_KERNEL_W, IGD_F_WALK_SERIAL; any other
+                                    bit (IGD_F_REF_QUIRKS included) is IGD_EINVAL  */
     int32_t arb_mode;            /* IGD_ARB_*                                     */
     int32_t tick_ms;             /* 20                                            */
     int32_t r2s_period_ms;       /* 200                                           */
     int32_t wd_ticks;            /* watchdog every wd_ticks ticks, 0 = never      */
-    int32_t frame0;
+    int32_t frame0;              /* index of this call's first tick (watchdog phase), >= 0 */
     int32_t reserved;
     int64_t now_ms0;
     /* receive side */
